@@ -2,6 +2,7 @@
 """bench.py — RTF / mel-frames-per-second of the F5-TTS ODE-sampling hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload cfg2|cfg3|cfg4|cfg5]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 One "step" = one pass of the hot path over one batch of synthetic utterances:
@@ -394,6 +395,20 @@ def parity_vs_reference(model, dev):
                 passed=bool(all(v <= 5e-3 for v in drift.values())))
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each tensor as out_dir/<name>.npy in float32 (every workload's outputs fit DUMP_LIMIT whole)."""
+    host = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
+
+
 def timed(fn, steps, warmup, barrier):
     for _ in range(warmup):
         fn()
@@ -534,7 +549,12 @@ def main():
     ap.add_argument("--workload", default="cfg2", choices=sorted(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the cfg3/cfg4/cfg5 records and the per-kernel tables")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (rank 0's mel and audio) as "
+                         "DIR/<name>.npy in float32; the inputs are seeded, so two builds can be compared output by output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     w = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -598,12 +618,15 @@ def main():
         barrier()
         e0.record()
         for _ in range(args.steps):
-            gather(*hot_path(model, voc, wav_d, text_d, dur_d, lens_d, nfe, w['frames'][0]))
+            last = hot_path(model, voc, wav_d, text_d, dur_d, lens_d, nfe, w['frames'][0])
+            gather(*last)
         e1.record()
         barrier()
     launches = _lib.launch_count() - l0
     ms = e0.elapsed_time(e1) / args.steps
     clocks = cs.summary()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(("mel", "audio"), last)))
 
     # ---- end to end through the reference-facing call with HOST buffers ---------------------------------------
     if w["B"] == 1:

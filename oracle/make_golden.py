@@ -180,6 +180,40 @@ def vocos_golden():
     np.savez_compressed(os.path.join(GOLD, "vocos_oracle_frozen.npz"), mel=mel.numpy(), wav=wav.numpy())
 
 
+def ref_tiny_b2_golden():
+    """Batch of two without prompt lengths (`lens` defaults to the full cond), seeded inputs; the reference's output is
+    kept so the oracle is compared with it wherever the tests run."""
+    cfg = tiny_dit()
+    sd = O.synthetic_state_dict(cfg, seed=1)
+    model = build_reference(cfg, sd)
+    g = torch.Generator().manual_seed(0)
+    cond = torch.randn(2, 20, 100, generator=g)
+    text = torch.randint(0, 50, (2, 25), generator=g)
+    dur = torch.tensor([60, 44])
+    with torch.no_grad():
+        out, _ = model.sample(cond=cond, text=text, duration=dur, steps=3, cfg_strength=2.0, sway_sampling_coef=-1.0,
+                              seed=1)
+    res = O.sample(sd, cfg, cond, text, dur, steps=3, cfg_strength=2.0, sway_sampling_coef=-1.0, seed=1)
+    print("[ref_tiny_b2] oracle-vs-ref rel-L2", rel_l2(res.out, out))
+    np.savez_compressed(os.path.join(GOLD, "ref_tiny_b2_nolens.npz"), cond=cond.numpy(), text=text.numpy(),
+                        duration=dur.numpy(), out=out.numpy())
+
+
+def model_configs_golden():
+    """The `model` section of the reference's configs/<name>.yaml for every model api.MODEL_ARCH restates."""
+    import json
+
+    import yaml
+
+    from f5_tts_b200 import api
+
+    cfg_dir = os.path.join(ref_shims.REFERENCE_SRC, "f5_tts", "configs")
+    table = {name: yaml.safe_load(open(os.path.join(cfg_dir, name + ".yaml")))["model"] for name in sorted(api.MODEL_ARCH)}
+    with open(os.path.join(GOLD, "model_configs.json"), "w") as f:
+        json.dump(table, f, indent=1, sort_keys=True)
+        f.write("\n")
+
+
 def main():
     os.makedirs(GOLD, exist_ok=True)
     torch.set_num_threads(os.cpu_count() or 8)
@@ -187,6 +221,8 @@ def main():
     istft_golden()
     vocos_golden()
     per_op_goldens()
+    model_configs_golden()
+    ref_tiny_b2_golden()
     # tiny end-to-end cases: every branch of sample()
     run_case("dit_tiny_b1_wave", tiny_dit(), B=1, n_ref=20, nt=24, durations=64, steps=4, cfg_strength=2.0,
              sway=-1.0, seed=3, wave=True)

@@ -160,19 +160,18 @@ def test_infer_process_empty_text(tmp_path):
     assert wav is None and spec is None and got_sr == sr
 
 
-def test_api_model_table_matches_reference_configs():
-    """api.MODEL_ARCH restates configs/*.yaml `model.arch` (hydra is not installed here); pinned against the reference's
-    own files when the reference tree is present (it is not on the GPU box)."""
-    import yaml
+def test_api_model_table_matches_reference_configs(golden_dir):
+    """api.MODEL_ARCH restates configs/*.yaml `model.arch` (hydra is not installed here); pinned against the `model`
+    sections of the reference's own files (model_configs.json, written by oracle/make_golden.py)."""
+    import json
 
     from f5_tts_b200 import api
     from f5_tts_b200.model import UNetT
 
-    cfg_dir = "/root/reference/src/f5_tts/configs"
-    if not os.path.isdir(cfg_dir):
-        pytest.skip("reference tree not present (GPU box)")
+    with open(os.path.join(golden_dir, "model_configs.json")) as f:
+        ref_configs = json.load(f)
     for name, (cls, arch) in api.MODEL_ARCH.items():
-        ref = yaml.safe_load(open(os.path.join(cfg_dir, name + ".yaml")))["model"]
+        ref = ref_configs[name]
         assert ref["backbone"] == cls.__name__ and (cls is UNetT) == (ref["backbone"] == "UNetT")
         ref_arch = {k: v for k, v in ref["arch"].items() if k != "checkpoint_activations"}  # training-only switch
         assert {k: arch[k] for k in ref_arch if k in arch} == {k: v for k, v in ref_arch.items() if k in arch}, name
