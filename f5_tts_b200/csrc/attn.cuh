@@ -220,7 +220,7 @@ attn_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmQKV, const AttnPar
   const uint32_t tmem_base = *tmem_slot;
   pdl_wait();
   pdl_launch_dependents();
-  // a sample always has at least one key: kv_len < 1 (caller error on the public entry point) is treated as 1
+  // kv_len[b] >= 1 here: a sample with kv_len[b] < 1 (a caller error) left above without writing any output
   const int kv_len = p.kv_len ? max(1, min(p.kv_len[b], p.seq)) : p.seq;
   const int n_kv = (kv_len + kAttnBKV - 1) / kAttnBKV;
 

@@ -304,8 +304,36 @@ int gemm_plan(GemmPlan* pl, const void* A, const void* W, const f5_gemm_args* a)
     set_error("gemm: empty problem (rows=%d batches=%d n_out=%d)", a->rows, a->batches, a->n_out);
     return -1;
   }
-  if (a->epi == F5_EPI_QKV_ROPE && (a->inner % 64 || a->rope_cos == nullptr || a->seq <= 0)) {
+  // every argument is validated before the first driver call (tensor-map encoding), so a bad layout is reported as such
+  if (a->epi == F5_EPI_QKV_ROPE && (a->inner % 64 || a->rope_cos == nullptr || a->rope_sin == nullptr || a->seq <= 0)) {
     set_error("gemm: QKV_ROPE needs inner %% 64 == 0, rope tables and seq");
+    return -1;
+  }
+  if (conv) {
+    if (a->n_out % 64 || a->lda < a->n_out) {
+      set_error("conv gemm: channels must be a multiple of 64 (got %d, lda %d)", a->n_out, a->lda);
+      return -1;
+    }
+  } else if (a->k <= 0 || a->lda < a->k || a->ldw < a->k) {
+    set_error("gemm: bad k/lda/ldw (%d, %d, %d)", a->k, a->lda, a->ldw);
+    return -1;
+  }
+  if (a->epi == F5_EPI_F32) {
+    if (a->out == nullptr || (reinterpret_cast<uintptr_t>(a->out) & 15)) {
+      set_error("gemm: fp32 epilogue needs a 16-byte aligned out (out=%p)", a->out);
+      return -1;
+    }
+    if (a->out16b != nullptr && ((reinterpret_cast<uintptr_t>(a->out16b) & 15) || a->ldo % 8)) {
+      set_error("gemm: out16b needs a 16-byte aligned pointer and ldo %% 8 == 0 (out16b=%p ldo=%d)", a->out16b, a->ldo);
+      return -1;
+    }
+  } else if (a->epi == F5_EPI_RESID) {
+    if (a->ldo % 4 || a->resid == nullptr) {
+      set_error("gemm: RESID epilogue needs resid != NULL and ldo %% 4 == 0 (ldo=%d)", a->ldo);
+      return -1;
+    }
+  } else if (a->ldo % 8 || a->out == nullptr) {
+    set_error("gemm: fp16 epilogue needs out != NULL and ldo %% 8 == 0 (ldo=%d)", a->ldo);
     return -1;
   }
   pl->bn = bn;
@@ -347,10 +375,6 @@ int gemm_plan(GemmPlan* pl, const void* A, const void* W, const f5_gemm_args* a)
 #endif
   int rc;
   if (conv) {
-    if (a->n_out % 64 || a->lda < a->n_out) {
-      set_error("conv gemm: channels must be a multiple of 64 (got %d, lda %d)", a->n_out, a->lda);
-      return -1;
-    }
     p.num_kb = a->conv_taps;
     // activations [batches][rows][lda]: channel slice of 64 = one group
     rc = encode_tmap_f16(&pl->tmA, A, (uint64_t)a->lda, (uint64_t)a->rows, (uint64_t)a->batches, (uint64_t)a->lda * 2,
@@ -359,10 +383,6 @@ int gemm_plan(GemmPlan* pl, const void* A, const void* W, const f5_gemm_args* a)
     rc = encode_tmap_f16(&pl->tmB, W, 64, (uint64_t)a->conv_taps * a->n_out, 1, 128, 0, 64, 64, 2);
     if (rc) return rc;
   } else {
-    if (a->k <= 0 || a->lda < a->k || a->ldw < a->k) {
-      set_error("gemm: bad k/lda/ldw (%d, %d, %d)", a->k, a->lda, a->ldw);
-      return -1;
-    }
     p.num_kb = (a->k + kBK - 1) / kBK;
     rc = encode_tmap_f16(&pl->tmA, A, (uint64_t)a->k, (uint64_t)a->rows, (uint64_t)a->batches, (uint64_t)a->lda * 2,
                          (uint64_t)a->rows * a->lda * 2, 64, 128, 3);
@@ -375,18 +395,10 @@ int gemm_plan(GemmPlan* pl, const void* A, const void* W, const f5_gemm_args* a)
   if (a->epi == F5_EPI_F32) {
     pl->tmC = pl->tmA;  // unused
   } else if (a->epi == F5_EPI_RESID) {
-    if (a->ldo % 4 || a->resid == nullptr) {
-      set_error("gemm: RESID epilogue needs resid != NULL and ldo %% 4 == 0 (ldo=%d)", a->ldo);
-      return -1;
-    }
     rc = encode_tmap(&pl->tmC, 1, a->resid, (uint64_t)a->n_out, (uint64_t)a->rows, (uint64_t)a->batches,
                      (uint64_t)a->ldo * 4, (uint64_t)a->rows * a->ldo * 4, 32, 128, 3);
     if (rc) return rc;
   } else {
-    if (a->ldo % 8 || a->out == nullptr) {
-      set_error("gemm: fp16 epilogue needs out != NULL and ldo %% 8 == 0 (ldo=%d)", a->ldo);
-      return -1;
-    }
     rc = encode_tmap(&pl->tmC, 0, a->out, (uint64_t)a->n_out, (uint64_t)a->rows, (uint64_t)a->batches,
                      (uint64_t)a->ldo * 2, (uint64_t)a->rows * a->ldo * 2, 64, 128, 3);
     if (rc) return rc;

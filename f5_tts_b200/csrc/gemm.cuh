@@ -142,8 +142,10 @@ __device__ __forceinline__ void epilogue_chunk(const GemmParams& p, const uint32
         }
       } else {
 #pragma unroll
-        for (int i = 0; i < 32; i += 2)
-          if (nc + i < p.n_out) *reinterpret_cast<uint32_t*>(o2 + i) = valid ? pack_half2(v[i], v[i + 1]) : 0u;
+        for (int i = 0; i < 32; i += 2) {
+          if (nc + i + 1 < p.n_out) *reinterpret_cast<uint32_t*>(o2 + i) = valid ? pack_half2(v[i], v[i + 1]) : 0u;
+          else if (nc + i < p.n_out) o2[i] = __float2half_rn(valid ? v[i] : 0.0f);  // odd n_out: column n_out is not ours
+        }
       }
     }
   } else if (EPI == EPI_RESID) {

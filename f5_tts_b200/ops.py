@@ -28,45 +28,60 @@ def _need_cuda(*ts):
             raise _lib.F5LibraryError("B200 operators take CUDA tensors only; there is no CPU fallback")
 
 
+def _rows(t: torch.Tensor, shape, dtype, what: str) -> int:
+    """Row stride of a caller-provided 2-D operand whose rows are contiguous (it may be a column slice)."""
+    assert t.shape == shape and t.dtype == dtype and t.stride(1) == 1, (what, t.shape, t.dtype, t.stride())
+    return t.stride(0)
+
+
 def linear(a: torch.Tensor, w: torch.Tensor, bias=None, *, epi=EPI_F16, act=ACT_NONE, bn=0, pair=0, resid=None, gate=None,
-           row_len=None, seq=0, rope=None, inner=0, pe_heads=0, out16b=False, static_w=False):
-    """C = epilogue(a @ w.T).  a fp16 [M, K], w fp16 [N, K] (both contiguous).
+           row_len=None, seq=0, rope=None, inner=0, pe_heads=0, out16b=False, static_w=False, out=None,
+           skip_padded=False, step_ptr=None, gate_stride=0):
+    """C = epilogue(a @ w.T).  a fp16 [M, K], w fp16 [N, K]; each may be row-strided (a column slice of a wider tensor).
     static_w: w is a model weight (not produced by the preceding kernel) -> its tiles may be prefetched early.
+    out: caller-allocated output [M, N] (fp16, or fp32 for EPI_F32), row-strided like a; allocated when None.
+    out16b (EPI_F32): True allocates the masked fp16 copy, a tensor is used as it (same row stride as out).
+    skip_padded: tiles whose rows all lie past row_len of their sample are not computed (needs row_len and seq).
+    step_ptr / gate_stride: the RESID gate row is gate + (*step_ptr) * gate_stride (device int32 step counter).
 """
-    _need_cuda(a, w, bias, resid, gate)
-    assert a.dtype == torch.float16 and w.dtype == torch.float16 and a.is_contiguous() and w.is_contiguous()
+    _need_cuda(a, w, bias, resid, gate, out, step_ptr)
     M, K = a.shape
     N = w.shape[0]
     g = _lib.GemmArgs()
-    g.rows, g.batches, g.n_out, g.k, g.lda, g.ldw, g.bn, g.epi, g.act = M, 1, N, K, a.stride(0), w.stride(0), bn, epi, act
+    g.rows, g.batches, g.n_out, g.k, g.bn, g.epi, g.act = M, 1, N, K, bn, epi, act
+    g.lda = _rows(a, (M, K), torch.float16, "a")
+    g.ldw = _rows(w, (N, K), torch.float16, "w")
     g.cta_pair = pair
     g.bias = _ptr(bias)
-    out = None
     out2 = None
-    if epi in (EPI_F16, EPI_QKV_ROPE):
-        out = torch.empty((M, N), dtype=torch.float16, device=a.device)
-        g.out = out.data_ptr()
-    elif epi == EPI_F32:
-        out = torch.empty((M, N), dtype=torch.float32, device=a.device)
-        g.out = out.data_ptr()
-        if out16b:
-            out2 = torch.empty((M, N), dtype=torch.float16, device=a.device)
-            g.out16b = out2.data_ptr()
-    else:
-        assert resid is not None and resid.dtype == torch.float32 and resid.is_contiguous()
+    if epi == EPI_RESID:
+        assert resid is not None and out is None
         out = resid
+        g.ldo = _rows(resid, (M, N), torch.float32, "resid")
         g.resid = resid.data_ptr()
-    g.ldo = N
+    else:
+        dt = torch.float32 if epi == EPI_F32 else torch.float16
+        if out is None:
+            out = torch.empty((M, N), dtype=dt, device=a.device)
+        g.ldo = _rows(out, (M, N), dt, "out")
+        g.out = out.data_ptr()
+        if epi == EPI_F32 and out16b is not False:
+            out2 = torch.empty((M, N), dtype=torch.float16, device=a.device) if out16b is True else out16b
+            assert _rows(out2, (M, N), torch.float16, "out16b") == g.ldo
+            g.out16b = out2.data_ptr()
     g.gate = _ptr(gate)
+    g.step_ptr = _ptr(step_ptr)
+    g.gate_step_stride = gate_stride
     g.row_len = _ptr(row_len)
     g.seq = seq
+    g.skip_padded_tiles = 1 if skip_padded else 0
     if rope is not None:
         g.rope_cos, g.rope_sin = rope[0].data_ptr(), rope[1].data_ptr()
     g.inner, g.pe_heads = inner, pe_heads
     g.weights_static = 1 if static_w else 0
     with torch.cuda.device(a.device):
         _lib.check(_lib.lib().f5_gemm(a.data_ptr(), w.data_ptr(), C.byref(g), _stream(a)), "f5_gemm")
-    return (out, out2) if out16b else out
+    return (out, out2) if out2 is not None else out
 
 
 def gemm_tile(M: int, N: int, K: int, epi=EPI_F16, act=ACT_NONE, bn=0, pair=0):
@@ -78,18 +93,23 @@ def gemm_tile(M: int, N: int, K: int, epi=EPI_F16, act=ACT_NONE, bn=0, pair=0):
     return b.value, pr.value
 
 
-def grouped_conv31(x: torch.Tensor, w_packed: torch.Tensor, bias, *, resid=None, row_len=None):
+def grouped_conv31(x: torch.Tensor, w_packed: torch.Tensor, bias, *, resid=None, row_len=None, out=None,
+                   skip_padded=False):
     """Conv1d(k=31, groups=D/64, pad=15) + bias + (mask) + Mish over x fp16 [B, N, D]; w_packed fp16 [31, D, 64].
-    resid given: resid += result (fp32, in place) else returns fp16 [B, N, D]."""
-    _need_cuda(x, w_packed, bias)
+    resid given: resid += result (fp32, in place) else returns fp16 [B, N, D] (into `out` when given, contiguous).
+    skip_padded: 128-row tiles starting at or past row_len[b] are not computed."""
+    _need_cuda(x, w_packed, bias, resid, row_len, out)
     B, N, D = x.shape
     g = _lib.GemmArgs()
     g.rows, g.batches, g.n_out, g.lda, g.conv_taps, g.act = N, B, D, D, 31, ACT_MISH
     g.bias = _ptr(bias)
     g.ldo, g.seq, g.row_len = D, N, _ptr(row_len)
+    g.skip_padded_tiles = 1 if skip_padded else 0
     g.weights_static = 1
     if resid is None:
-        out = torch.empty((B, N, D), dtype=torch.float16, device=x.device)
+        if out is None:
+            out = torch.empty((B, N, D), dtype=torch.float16, device=x.device)
+        assert out.shape == (B, N, D) and out.dtype == torch.float16 and out.is_contiguous()
         g.epi, g.out = EPI_F16, out.data_ptr()
     else:
         out = resid
@@ -99,11 +119,14 @@ def grouped_conv31(x: torch.Tensor, w_packed: torch.Tensor, bias, *, resid=None,
     return out
 
 
-def attention(qkv: torch.Tensor, batches: int, seq: int, heads: int, kv_len=None, scale=None) -> torch.Tensor:
-    """qkv fp16 [batches*seq, 3*heads*64] -> fp16 [batches*seq, heads*64]"""
-    _need_cuda(qkv, kv_len)
+def attention(qkv: torch.Tensor, batches: int, seq: int, heads: int, kv_len=None, scale=None, out=None) -> torch.Tensor:
+    """qkv fp16 [batches*seq, 3*heads*64] -> fp16 [batches*seq, heads*64] (into `out` when given, contiguous).
+    With kv_len, query blocks of 256 rows at or past kv_len[b] are not written."""
+    _need_cuda(qkv, kv_len, out)
     assert qkv.dtype == torch.float16 and qkv.is_contiguous() and qkv.shape == (batches * seq, 3 * heads * 64)
-    out = torch.empty((batches * seq, heads * 64), dtype=torch.float16, device=qkv.device)
+    if out is None:
+        out = torch.empty((batches * seq, heads * 64), dtype=torch.float16, device=qkv.device)
+    assert out.shape == (batches * seq, heads * 64) and out.dtype == torch.float16 and out.is_contiguous()
     scale = 0.125 if scale is None else scale
     with torch.cuda.device(qkv.device):
         _lib.check(_lib.lib().f5_attention(qkv.data_ptr(), out.data_ptr(), batches, seq, heads, _ptr(kv_len), scale,

@@ -56,10 +56,11 @@ typedef struct {
   int conv_taps; /* 0 = plain GEMM */
   int cta_pair;  /* 1 = 2-CTA (cta_group::2) 256 x bn tiles; bn must be 128 or 256; plain GEMM, not EPI_F32 */
   const float* bias;
-  void* out;               /* fp16 (F16 / QKV_ROPE) or fp32 (F32) [batches*rows, ldo] */
-  void* out16b;            /* optional fp16 masked copy for F32 */
-  float* resid;            /* RESID: in/out fp32 */
-  int ldo;
+  void* out;               /* fp16 (F16 / QKV_ROPE, ldo % 8 == 0) or fp32 (F32, 16-byte aligned) [batches*rows, ldo] */
+  void* out16b;            /* optional fp16 masked copy for F32 (rows past row_len are 0), same ldo: needs a 16-byte
+                              aligned pointer and ldo % 8 == 0 */
+  float* resid;            /* RESID: in/out fp32, ldo % 4 == 0 */
+  int ldo;                 /* output row stride in elements (>= n_out); columns n_out .. ldo-1 are never written */
   const float* gate;       /* RESID: per-column gate (NULL = 1) */
   const int* step_ptr;     /* device step counter used to index gate (NULL = 0) */
   long long gate_step_stride;
@@ -81,7 +82,10 @@ int f5_gemm_tile(const f5_gemm_args* args, int* bn, int* cta_pair);
 
 /* Non-causal attention over the fused QKV buffer — replaces F.scaled_dot_product_attention at
  * model/modules.py:519 (attn_mask=None, or the key mask of modules.py:513-517 via kv_len).
- *   qkv fp16 [batches*seq, 3*heads*64]; out fp16 [batches*seq, heads*64]. dim_head must be 64. */
+ *   qkv fp16 [batches*seq, 3*heads*64]; out fp16 [batches*seq, heads*64]. dim_head must be 64.
+ *   kv_len (device int32 [batches] or NULL = seq): sample b attends to its first kv_len[b] keys; 1 <= kv_len[b] is
+ *   required.  With kv_len, the 256-row query blocks of sample b that start at or past kv_len[b] are not written (those
+ *   rows of out keep what the buffer held; kv_len[b] = 0 leaves the whole sample unwritten). */
 int f5_attention(const void* qkv, void* out, int batches, int seq, int heads, const int* kv_len, float scale,
                  f5_stream_t stream);
 

@@ -87,3 +87,45 @@ def test_gemm_tile_planner():
             assert bn != 192 and not pair  # only instantiated shapes are ever chosen
     assert ops.gemm_tile(1876, 1024, 1024, EPI_RESID, ACT_NONE, bn=64) == (64, 0)  # explicit request is kept
     assert ops.gemm_tile(15008, 3072, 1024, EPI_QKV_ROPE, ACT_NONE) == (256, 1)  # large batch: cta_group::2 pairs
+
+
+_FAKE_A, _FAKE_W, _FAKE_OUT, _FAKE_OUT2 = 0x7f0000000000, 0x7f0000100000, 0x7f0000200000, 0x7f0000300000
+
+
+@pytest.mark.parametrize("case,want", [
+    ("out16b_odd_ldo", "out16b"),      # F32 + out16b, ldo = n_out = 101: the fp16 copy's pair stores need ldo % 8 == 0
+    ("f32_out_misaligned", "aligned out"),  # F32 full chunks are float4 stores
+    ("f16_ldo", "ldo % 8"),            # fp16 TMA store rows must be 16-byte aligned
+    ("resid_null", "resid != NULL"),
+    ("qkv_no_tables", "rope tables"),
+    ("lda_lt_k", "lda"),
+])
+def test_gemm_rejects_bad_layout_before_driver(case, want):
+    """gemm_plan validates every argument before it encodes a tensor map, so a bad layout is reported as itself (never as
+    a driver error, and identically with or without a GPU).  The pointers are fake: rejected calls never dereference them."""
+    import ctypes as C
+
+    from f5_tts_b200 import _lib
+    from f5_tts_b200.ops import EPI_F16, EPI_F32, EPI_QKV_ROPE, EPI_RESID
+
+    if not os.path.exists(_lib.LIB_PATH):
+        pytest.skip("library not built (run __graft_entry__.build())")
+    g = _lib.GemmArgs()
+    g.rows, g.batches, g.n_out, g.k, g.lda, g.ldw, g.bn, g.epi = 256, 1, 256, 128, 128, 128, 128, EPI_F16
+    g.out, g.ldo = _FAKE_OUT, 256
+    if case == "out16b_odd_ldo":
+        g.epi, g.n_out, g.ldo, g.out16b = EPI_F32, 101, 101, _FAKE_OUT2
+    elif case == "f32_out_misaligned":
+        g.epi, g.out = EPI_F32, _FAKE_OUT + 4
+    elif case == "f16_ldo":
+        g.n_out, g.ldo = 100, 100
+    elif case == "resid_null":
+        g.epi, g.out = EPI_RESID, None
+    elif case == "qkv_no_tables":
+        g.epi, g.n_out, g.ldo, g.inner, g.seq = EPI_QKV_ROPE, 384, 384, 128, 128
+    elif case == "lda_lt_k":
+        g.lda = 64
+    lib = _lib.lib()
+    rc = lib.f5_gemm(_FAKE_A, _FAKE_W, C.byref(g), None)
+    msg = lib.f5_last_error().decode()
+    assert rc < 0 and want in msg and "cuTensorMap" not in msg, (rc, msg)
