@@ -17,6 +17,8 @@ c_void_p, c_int, c_float, c_size_t, c_ll = C.c_void_p, C.c_int, C.c_float, C.c_s
 
 ACT_NONE, ACT_GELU_TANH, ACT_GELU_ERF, ACT_MISH = 0, 1, 2, 3
 EPI_F16, EPI_F32, EPI_RESID, EPI_QKV_ROPE = 0, 1, 2, 3
+ODE_EULER, ODE_MIDPOINT = 0, 1
+ODE_METHODS = {"euler": ODE_EULER, "midpoint": ODE_MIDPOINT}
 
 
 class GemmArgs(C.Structure):
@@ -73,7 +75,7 @@ class SampleArgs(C.Structure):
         ("B", c_int), ("N", c_int), ("nt", c_int), ("steps", c_int),
         ("text", c_void_p), ("step_cond", c_void_p), ("y", c_void_p), ("duration", c_void_p),
         ("t", C.POINTER(c_float)), ("cfg_strength", c_float), ("trajectory", c_void_p), ("use_graph", c_int),
-        ("v_out", c_void_p), ("exact_varlen", c_int),
+        ("v_out", c_void_p), ("exact_varlen", c_int), ("ode_method", c_int),
     ]
 
 

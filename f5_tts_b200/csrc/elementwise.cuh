@@ -1,5 +1,5 @@
 // Bandwidth-bound kernels of the ODE-sampling path: row normalisations (+AdaLN modulation), depthwise conv + LN,
-// text embedding gather, GRN, input packing, CFG + Euler update, small fp32 linears, rotary tables.
+// text embedding gather, GRN, input packing, CFG + ODE update, small fp32 linears, rotary tables.
 // All are warp-per-row / grid-stride kernels with 128-bit vectorised, coalesced global accesses.
 #pragma once
 #include "common.cuh"
@@ -241,7 +241,7 @@ __global__ void grn_apply_kernel(__half* g, const float* nx, const float* gamma,
 
 // ---------------------------------------------------------------------------------------------------------
 // Input packing (backbones/dit.py:151-163): xin[Be*N, Kpad] fp16 = [ x | cond or 0 | text_emb | 0-pad ].
-// Static part once per sample(); the x columns are rewritten every step by the Euler kernel.
+// Static part once per sample(); the x columns are rewritten after every evaluation by the update kernel.
 // ---------------------------------------------------------------------------------------------------------
 
 __global__ void pack_input_kernel(const PackParams p) {
@@ -259,17 +259,19 @@ __global__ void pack_input_kernel(const PackParams p) {
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// CFG + Euler (cfm.py:190-191 + torchdiffeq fixed-grid Euler, cfm.py:218):
-//   y <- y + dt[k] * (pred + (pred - null) * cfg);  trajectory[k+1] = y;  xin[:, :mel] <- fp16(y) for both halves;
-//   the last thread-block-0 thread advances the device step counter so one captured graph serves every step.
+// CFG + ODE update (cfm.py:190-191 + torchdiffeq fixed-grid Euler / midpoint, cfm.py:218), one launch per backbone
+// evaluation e = *step_ptr with st = stages[e] (ew_params.h: OdeStage):
+//   x = y + st.coef * (pred + (pred - null) * cfg);  xin[:, :mel] <- fp16(x) for both halves;
+//   st.commit >= 0: y <- x, trajectory[st.commit] = x;
+//   the last thread block to finish advances the device counter so one captured graph serves every evaluation.
 // v: [Be*N, mel] fp32 (pred rows first, null rows second).
 // ---------------------------------------------------------------------------------------------------------
 
-__global__ void cfg_euler_kernel(const EulerParams p) {
+__global__ void cfg_update_kernel(const UpdateParams p) {
   pdl_wait();
   pdl_launch_dependents();
-  const int k = *p.step_ptr;
-  const float dt = p.dt[k];
+  const int e = *p.step_ptr;
+  const OdeStage st = p.stages[e];
   const SampleIo io = *p.io;
   const long long total = (long long)p.BN * p.mel;
   const long long null_off = (long long)p.B * p.seq_tok * p.mel;
@@ -285,21 +287,23 @@ __global__ void cfg_euler_kernel(const EulerParams p) {
       const float nu = p.v[null_off + vi];
       g = pr + (pr - nu) * io.cfg;
     }
-    const float yn = io.y[i] + dt * g;
-    io.y[i] = yn;
-    if (io.traj) io.traj[(long long)(k + 1) * total + i] = yn;
-    const __half h = __float2half_rn(yn);
+    const float x = io.y[i] + st.coef * g;
+    if (st.commit >= 0) {
+      io.y[i] = x;
+      if (io.traj) io.traj[(long long)st.commit * total + i] = x;
+    }
+    const __half h = __float2half_rn(x);
     p.xin[r * p.Kpad + c] = h;
     if (p.packed) p.xin[(r + p.BN) * p.Kpad + c] = h;
   }
-  // the last CTA to finish advances the device step counter (every CTA has read step k by then)
+  // the last CTA to finish advances the device counter (every CTA has read entry e by then)
   __syncthreads();
   if (threadIdx.x == 0) {
     __threadfence();
     int* done = p.step_ptr + 1;
     if (atomicAdd(done, 1) == int(gridDim.x) - 1) {
       *done = 0;
-      *p.step_ptr = k + 1;
+      *p.step_ptr = e + 1;
     }
   }
 }

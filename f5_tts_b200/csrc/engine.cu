@@ -3,13 +3,16 @@
 //
 // Per sample() call (hoisted out of the NFE loop because it is step- or batch-invariant):
 //   * text embeddings, cond + uncond variants (dit.py:284-314 caches them the same way)
-//   * time embedding of every grid point and — DiT — the AdaLN modulation vectors of every (step, block)
-//     as one [steps, depth*6D + 2D] table: 22 weight-streaming GEMVs per step become one GEMM per call
+//   * time embedding of every backbone evaluation and — DiT — the AdaLN modulation vectors of every (evaluation,
+//     block) as one [evals, depth*6D + 2D] table: 22 weight-streaming GEMVs per evaluation become one GEMM per call
+//     (evals = steps for Euler, 2 * steps for midpoint: every table is indexed by evaluation, not by grid step)
 //   * rotary cos/sin table, static columns of the packed input projection operand
-// Per NFE step: input projection -> grouped conv position embedding x2 (tensor-core implicit GEMM) -> depth x
+// Per backbone evaluation: input projection -> grouped conv position embedding x2 (tensor-core implicit GEMM) -> depth x
 // {norm+modulate, fused QKV+RoPE GEMM, flash attention, out-proj (+gate, +mask, +residual), norm+modulate,
-//  FF1+GELU, FF2 (+gate, +residual)} -> final norm -> proj_out -> fused CFG + Euler update.
-// Every kernel reads the step index from a device counter, so one captured CUDA graph serves all steps.
+//  FF1+GELU, FF2 (+gate, +residual)} -> final norm -> proj_out -> fused CFG + ODE update (Euler step, midpoint half
+// step or midpoint full step, read from the per-evaluation OdeStage table).
+// Every kernel reads the evaluation index from a device counter, so one captured CUDA graph serves all evaluations.
+#include <climits>
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
@@ -37,13 +40,13 @@ struct Bump {
 
 struct Layout {
   // sizes
-  int B, Be, N, seq, steps, packed;
+  int B, Be, N, seq, evals, packed;  // evals: backbone evaluations of the call (ode_evals)
   long long M, M1;
   // common
   int* step_ptr;
   SampleIo* io;     // caller tensors + cfg scale of THIS call, read by the step kernels through the workspace
-  float* dt;
-  float* t_dev;
+  OdeStage* stages;  // [evals]
+  float* t_dev;      // [evals] time of every evaluation
   float *rope_cos, *rope_sin;
   int* row_len;     // [Be] or unused
   int* kv_len;      // [Be] or unused
@@ -87,9 +90,12 @@ struct GraphHolder {
 };
 struct GraphKey {
   const void* ws;
-  int B, N, steps, packed, masked;  // masked: 0 = no lengths, 1 = lengths (reference batched semantics), 2 = exact_varlen
+  // evals, not (steps, method): the layout and every kernel plan depend on the evaluation count only, and the solver's
+  // rule lives in the OdeStage table the prologue uploads per call — so an Euler call with 2S steps and a midpoint call
+  // with S steps share one graph.
+  int B, N, evals, packed, masked;  // masked: 0 = no lengths, 1 = lengths (reference batched semantics), 2 = exact_varlen
   bool operator==(const GraphKey& o) const {
-    return ws == o.ws && B == o.B && N == o.N && steps == o.steps && packed == o.packed && masked == o.masked;
+    return ws == o.ws && B == o.B && N == o.N && evals == o.evals && packed == o.packed && masked == o.masked;
   }
 };
 struct GraphEntry {
@@ -106,12 +112,14 @@ struct f5_engine {
   std::vector<GraphEntry> graphs;
 };
 
-static void plan_layout(const f5_engine* e, Layout& L, void* ws, int B, int N, int steps, float cfg) {
+static int ode_evals(int steps, int ode_method) { return ode_method == F5_ODE_MIDPOINT ? 2 * steps : steps; }
+
+static void plan_layout(const f5_engine* e, Layout& L, void* ws, int B, int N, int evals, float cfg) {
   const f5_arch& A = e->arch;
   Bump bp(ws);
   L.B = B;
   L.N = N;
-  L.steps = steps;
+  L.evals = evals;
   L.packed = cfg < 1e-5f ? 0 : 1;
   L.Be = L.packed ? 2 * B : B;
   L.seq = A.backbone == 1 ? N + 1 : N;
@@ -120,19 +128,19 @@ static void plan_layout(const f5_engine* e, Layout& L, void* ws, int B, int N, i
   const int D = A.dim, Td = A.text_dim, F = A.ff_inner;
   L.step_ptr = bp.take<int>(64);
   L.io = bp.take<SampleIo>(1);
-  L.dt = bp.take<float>(steps + 1);
-  L.t_dev = bp.take<float>(steps + 1);
+  L.stages = bp.take<OdeStage>(evals);
+  L.t_dev = bp.take<float>(evals);
   L.rope_cos = bp.take<float>((size_t)L.seq * 32);
   L.rope_sin = bp.take<float>((size_t)L.seq * 32);
   L.row_len = bp.take<int>(L.Be);
   L.kv_len = bp.take<int>(L.Be);
   L.frame_len = bp.take<int>(L.Be);
   L.valid_len = bp.take<int>(B);
-  L.tfeat = bp.take<float>((size_t)steps * 256);
-  L.th1 = bp.take<float>((size_t)steps * D);
-  L.temb = bp.take<float>((size_t)steps * D);
-  L.temb_silu = bp.take<__half>((size_t)steps * D);
-  L.mod = bp.take<float>((size_t)steps * (e->modW > 0 ? e->modW : 1));
+  L.tfeat = bp.take<float>((size_t)evals * 256);
+  L.th1 = bp.take<float>((size_t)evals * D);
+  L.temb = bp.take<float>((size_t)evals * D);
+  L.temb_silu = bp.take<__half>((size_t)evals * D);
+  L.mod = bp.take<float>((size_t)evals * (e->modW > 0 ? e->modW : 1));
   L.tx = bp.take<float>((size_t)2 * B * N * Td);
   L.filler = bp.take<uint8_t>((size_t)B * N);
   L.ta = bp.take<__half>((size_t)2 * B * N * Td);
@@ -207,13 +215,13 @@ void f5_engine_destroy(f5_engine* e) {
   delete e;  // graph holders destroy their executables
 }
 
-size_t f5_sample_workspace_bytes(const f5_engine* e, int B, int N, int steps, float cfg_strength) {
+size_t f5_sample_workspace_bytes(const f5_engine* e, int B, int N, int evals, float cfg_strength) {
   Layout L;
-  plan_layout(e, L, nullptr, B, N, steps, cfg_strength);
+  plan_layout(e, L, nullptr, B, N, evals, cfg_strength);
   return L.bytes;
 }
 
-double f5_sample_flops(const f5_engine* e, int B, int N, int steps, float cfg_strength) {
+double f5_sample_flops(const f5_engine* e, int B, int N, int evals, float cfg_strength) {
   const f5_arch& A = e->arch;
   const double D = A.dim, mel = A.mel_dim, Td = A.text_dim, F = A.ff_inner, Ld = A.depth;
   const double Be = cfg_strength < 1e-5f ? B : 2.0 * B;
@@ -227,11 +235,11 @@ double f5_sample_flops(const f5_engine* e, int B, int N, int steps, float cfg_st
     per = Ld * (8.0 * n1 * D * D + 4.0 * n1 * D * F + 4.0 * n1 * n1 * D) + (Ld / 2.0) * 4.0 * n1 * D * D +
           2.0 * n * (2 * mel + Td) * D + 2.0 * (2.0 * n * D * (D / 16.0) * 31.0) + 2.0 * n1 * D * mel;
   }
-  double total = steps * Be * per;
+  double total = evals * Be * per;
   // text embedding, once per sample and CFG branch: conv_layers x (2 pointwise GEMMs)
   total += 2.0 * B * A.conv_layers * (2.0 * 2.0 * N * Td * 2.0 * Td);
   // conditioning: time MLP + AdaLN table, once per call
-  total += steps * (2.0 * 256 * D + 2.0 * D * D + 2.0 * D * (double)e->modW);
+  total += evals * (2.0 * 256 * D + 2.0 * D * D + 2.0 * D * (double)e->modW);
   return total;
 }
 
@@ -475,11 +483,11 @@ int run_step(f5_engine* e, const Layout& L, const f5_sample_args* sa, const Step
     RC(norm_mod(e, L, L.x, L.M1, 2, e->w.g_out, nullptr, false, s));
   }
   RC(gemm_run(P.out_proj, s));
-  EulerParams ep{};
+  UpdateParams ep{};
   ep.io = L.io;
   ep.v = L.v;
   ep.xin = L.xin;
-  ep.dt = L.dt;
+  ep.stages = L.stages;
   ep.step_ptr = L.step_ptr;
   ep.BN = L.B * L.N;
   ep.mel = A.mel_dim;
@@ -489,21 +497,36 @@ int run_step(f5_engine* e, const Layout& L, const f5_sample_args* sa, const Step
   ep.seq_tok = L.seq;
   ep.tok_off = dit ? 0 : 1;
   ep.B = L.B;
-  return run_cfg_euler(ep, s);
+  return run_cfg_update(ep, s);
 }
 
 int run_prologue(f5_engine* e, const Layout& L, const f5_sample_args* sa, cudaStream_t s) {
   const f5_arch& A = e->arch;
   const f5_weights& W = e->w;
-  const int D = A.dim, Td = A.text_dim, B = L.B, N = L.N, S = L.steps;
+  const int D = A.dim, Td = A.text_dim, B = L.B, N = L.N, E = L.evals;
   const bool dit = A.backbone == 0;
   const bool masked = sa->duration != nullptr;
   const bool strict = masked && sa->exact_varlen;
+  // per-evaluation update rule and time, in fp32 as torchdiffeq forms them on the grid's dtype:
+  // Euler evaluates at t_k; midpoint at t_k and at t_k + dt/2 with dt = t_{k+1} - t_k
+  std::vector<OdeStage> stage(E);
+  std::vector<float> te(E);
+  for (int k = 0; k < sa->steps; ++k) {
+    const float dt = sa->t[k + 1] - sa->t[k];
+    if (sa->ode_method == F5_ODE_MIDPOINT) {
+      const float half = 0.5f * dt;
+      stage[2 * k] = OdeStage{half, -1};
+      stage[2 * k + 1] = OdeStage{dt, k + 1};
+      te[2 * k] = sa->t[k];
+      te[2 * k + 1] = sa->t[k] + half;
+    } else {
+      stage[k] = OdeStage{dt, k + 1};
+      te[k] = sa->t[k];
+    }
+  }
   // small host -> device control data (pageable source: cudaMemcpyAsync stages it before returning)
-  std::vector<float> dt(S + 1, 0.f);
-  for (int k = 0; k < S; ++k) dt[k] = sa->t[k + 1] - sa->t[k];
-  RC(check_cuda(cudaMemcpyAsync(L.dt, dt.data(), sizeof(float) * (S + 1), cudaMemcpyHostToDevice, s), "dt h2d"));
-  RC(check_cuda(cudaMemcpyAsync(L.t_dev, sa->t, sizeof(float) * (S + 1), cudaMemcpyHostToDevice, s), "t h2d"));
+  RC(check_cuda(cudaMemcpyAsync(L.stages, stage.data(), sizeof(OdeStage) * E, cudaMemcpyHostToDevice, s), "stages h2d"));
+  RC(check_cuda(cudaMemcpyAsync(L.t_dev, te.data(), sizeof(float) * E, cudaMemcpyHostToDevice, s), "t h2d"));
   RC(check_cuda(cudaMemsetAsync(L.step_ptr, 0, sizeof(int) * 64, s), "step memset"));
   SampleIo io{sa->y, sa->trajectory, sa->cfg_strength};
   RC(check_cuda(cudaMemcpyAsync(L.io, &io, sizeof(io), cudaMemcpyHostToDevice, s), "io h2d"));
@@ -530,13 +553,13 @@ int run_prologue(f5_engine* e, const Layout& L, const f5_sample_args* sa, cudaSt
     }
   }
   RC(run_rope_table(L.rope_cos, L.rope_sin, L.seq, 32, s));
-  // time embedding for every grid point (modules.py:852-862)
-  RC(run_time_features(L.t_dev, L.tfeat, S, 256, s));
-  RC(run_small_linear(1, L.tfeat, reinterpret_cast<const __half*>(W.time_w0), W.time_b0, L.th1, S, 256, D, s));
-  RC(run_small_linear(0, L.th1, reinterpret_cast<const __half*>(W.time_w1), W.time_b1, L.temb, S, D, D, s));
+  // time embedding for every backbone evaluation (modules.py:852-862)
+  RC(run_time_features(L.t_dev, L.tfeat, E, 256, s));
+  RC(run_small_linear(1, L.tfeat, reinterpret_cast<const __half*>(W.time_w0), W.time_b0, L.th1, E, 256, D, s));
+  RC(run_small_linear(0, L.th1, reinterpret_cast<const __half*>(W.time_w1), W.time_b1, L.temb, E, D, D, s));
   if (dit) {
-    RC(run_silu_to_half(L.temb, L.temb_silu, (long long)S * D, s));
-    f5_gemm_args a = base_args(S, e->modW, D, D, D, 128, F5_EPI_F32, F5_ACT_NONE);
+    RC(run_silu_to_half(L.temb, L.temb_silu, (long long)E * D, s));
+    f5_gemm_args a = base_args(E, e->modW, D, D, D, 128, F5_EPI_F32, F5_ACT_NONE);
     a.bias = W.mod_b;
     a.out = L.mod;
     a.ldo = e->modW;
@@ -631,15 +654,24 @@ extern "C" int f5_sample(f5_engine* e, const f5_sample_args* sa, void* workspace
     set_error("f5_sample: empty problem (B=%d N=%d steps=%d nt=%d)", sa->B, sa->N, sa->steps, sa->nt);
     return -1;
   }
+  if (sa->ode_method != F5_ODE_EULER && sa->ode_method != F5_ODE_MIDPOINT) {
+    set_error("f5_sample: ode_method must be F5_ODE_EULER (0) or F5_ODE_MIDPOINT (1) (got %d)", sa->ode_method);
+    return -1;
+  }
+  if (sa->ode_method == F5_ODE_MIDPOINT && sa->steps > INT_MAX / 2) {
+    set_error("f5_sample: steps=%d: 2 * steps midpoint evaluations overflow int", sa->steps);
+    return -1;
+  }
+  const int evals = ode_evals(sa->steps, sa->ode_method);
   Layout L;
-  plan_layout(e, L, workspace, sa->B, sa->N, sa->steps, sa->cfg_strength);
+  plan_layout(e, L, workspace, sa->B, sa->N, evals, sa->cfg_strength);
   if (ws_bytes < L.bytes) {
     set_error("f5_sample: workspace too small (%zu < %zu)", ws_bytes, L.bytes);
     return -1;
   }
   RC(run_prologue(e, L, sa, s));
   if (sa->use_graph) {
-    const GraphKey key{workspace, sa->B, sa->N, sa->steps, L.packed,
+    const GraphKey key{workspace, sa->B, sa->N, evals, L.packed,
                        sa->duration == nullptr ? 0 : (sa->exact_varlen ? 2 : 1)};
     std::shared_ptr<GraphHolder> g;
     {
@@ -682,12 +714,12 @@ extern "C" int f5_sample(f5_engine* e, const f5_sample_args* sa, void* workspace
       if (e->graphs.size() >= 16) e->graphs.erase(e->graphs.begin());  // holder is freed when its last user is done
       e->graphs.push_back(GraphEntry{key, g});
     }
-    for (int k = 0; k < sa->steps; ++k) RC(check_cuda(cudaGraphLaunch(g->exec, s), "graph launch"));
-    count_launch(g->nodes * sa->steps);
+    for (int k = 0; k < evals; ++k) RC(check_cuda(cudaGraphLaunch(g->exec, s), "graph launch"));
+    count_launch(g->nodes * evals);
     return copy_v_out(e, L, sa, s);
   }
   StepPlans P;
   RC(build_step_plans(e, L, sa, P));
-  for (int k = 0; k < sa->steps; ++k) RC(run_step(e, L, sa, P, s));
+  for (int k = 0; k < evals; ++k) RC(run_step(e, L, sa, P, s));
   return copy_v_out(e, L, sa, s);
 }

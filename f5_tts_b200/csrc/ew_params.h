@@ -56,11 +56,21 @@ struct SampleIo {
   float cfg;    // classifier-free-guidance scale
 };
 
-struct EulerParams {
+// One entry per backbone evaluation of a sample() call, indexed by the device counter.  The update kernel forms
+// x = y + coef * g (g: CFG-combined velocity) and writes fp16(x) into the next evaluation's input; commit >= 0 also stores
+// x as the ODE state y and as trajectory[commit], commit = -1 leaves y (the state at the start of the grid step) as it is.
+//   Euler:    {dt_k, k + 1}
+//   midpoint: {dt_k / 2, -1}, {dt_k, k + 1}   (torchdiffeq: y_mid = y + f0 * dt/2, y + dt * f(t_k + dt/2, y_mid))
+struct OdeStage {
+  float coef;
+  int commit;
+};
+
+struct UpdateParams {
   const SampleIo* io;
   const float* v;  // [Be*N, mel]
   __half* xin;
-  const float* dt;  // [steps] device
+  const OdeStage* stages;  // [evaluations] device
   int* step_ptr;
   int BN, mel, Kpad, packed;
   int N;         // frames per sample

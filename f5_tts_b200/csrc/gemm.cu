@@ -418,7 +418,7 @@ int gemm_plan(GemmPlan* pl, const void* A, const void* W, const f5_gemm_args* a)
 
 extern "C" {
 
-int f5_version(void) { return 100; }
+int f5_version(void) { return 101; }  // 101: f5_sample_args.ode_method
 const char* f5_last_error(void) { return f5::g_err; }
 unsigned long long f5_launch_count(void) { return f5::g_launches.load(); }
 

@@ -85,7 +85,7 @@ constexpr int kGrnRows = 64;  // sequence rows per partial-sum block
 int run_grn(__half* g, float* partial, float* nx, const float* gamma, const float* beta, int B, int N, int C,
             cudaStream_t s);
 int run_pack_input(const PackParams& p, cudaStream_t s);
-int run_cfg_euler(const EulerParams& p, cudaStream_t s);
+int run_cfg_update(const UpdateParams& p, cudaStream_t s);
 int run_small_linear(int act, const float* in, const __half* W, const float* bias, float* out, int S, int K, int Nout,
                      cudaStream_t s);
 int run_time_features(const float* t, float* feat, int S, int dim, cudaStream_t s);

@@ -163,12 +163,12 @@ int run_pack_input(const PackParams& p, cudaStream_t s) {
   return check_launch("pack_input_kernel");
 }
 
-int run_cfg_euler(const EulerParams& p, cudaStream_t s) {
+int run_cfg_update(const UpdateParams& p, cudaStream_t s) {
   const long long total = (long long)p.BN * p.mel;
   PdlLaunch L1(dim3(grid_for(total, 256, 148 * 4)), dim3(256), 0, s);
-  if (int rc = check_cuda(cudaLaunchKernelEx(&L1.cfg, cfg_euler_kernel, p), "cfg_euler launch")) return rc;
+  if (int rc = check_cuda(cudaLaunchKernelEx(&L1.cfg, cfg_update_kernel, p), "cfg_update launch")) return rc;
   count_launch(1);
-  return check_launch("cfg_euler_kernel");
+  return check_launch("cfg_update_kernel");
 }
 
 int run_small_linear(int act, const float* in, const __half* W, const float* bias, float* out, int S, int K, int Nout,

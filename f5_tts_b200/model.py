@@ -156,6 +156,19 @@ def _init_tensor(shape, how):
     return torch.randn(shape) / math.sqrt(max(fan_in, 1))
 
 
+def _ode_method_id(method: str) -> int:
+    """torchdiffeq method name -> f5_sample_args.ode_method; the engine builds the fixed-grid "euler" and "midpoint"."""
+    if method not in _lib.ODE_METHODS:
+        raise NotImplementedError(f"ODE method {method!r} is not built: the engine implements 'euler' (the shipped "
+                                  "default) and 'midpoint'")
+    return _lib.ODE_METHODS[method]
+
+
+def _ode_evals(steps: int, method_id: int) -> int:
+    """backbone evaluations of `steps` grid steps: the `evals` argument of f5_sample_workspace_bytes / f5_sample_flops"""
+    return 2 * steps if method_id == _lib.ODE_MIDPOINT else steps
+
+
 class _Backbone(nn.Module):
     """Shared implementation of the `transformer(...)` operator seam (SURVEY.md §8b)."""
 
@@ -253,15 +266,17 @@ class _Backbone(nn.Module):
             self._ws_free.setdefault((torch.device(device), int(stream)), []).append(ws)
 
     def run(self, y, step_cond, text, t_grid, duration, cfg_strength, trajectory=None, v_out=None, use_graph=True,
-            exact_varlen=False):
-        """One engine call = len(t_grid)-1 Euler steps.  All tensors on the CUDA device, fp32 / int64 / int32."""
+            exact_varlen=False, ode_method="euler"):
+        """One engine call = len(t_grid)-1 steps of the fixed-grid ODE solver `ode_method` ("euler": one backbone
+        evaluation per step, "midpoint": two).  All tensors on the CUDA device, fp32 / int64 / int32."""
         st = self.engine()
         L = _lib.lib()
         B, N, mel = y.shape
         steps = len(t_grid) - 1
         assert y.is_contiguous() and step_cond.is_contiguous() and text.is_contiguous()
         assert y.dtype == torch.float32 and step_cond.dtype == torch.float32 and text.dtype == torch.int64
-        need = L.f5_sample_workspace_bytes(st["handle"], B, N, steps, float(cfg_strength))
+        method = _ode_method_id(ode_method)
+        need = L.f5_sample_workspace_bytes(st["handle"], B, N, _ode_evals(steps, method), float(cfg_strength))
         stream = torch.cuda.current_stream(y.device).cuda_stream
         ws = self._ws_acquire(need, y.device, stream)
         tg = (C.c_float * (steps + 1))(*[float(v) for v in t_grid])
@@ -275,14 +290,16 @@ class _Backbone(nn.Module):
         a.use_graph = 1 if use_graph else 0
         a.v_out = v_out.data_ptr() if v_out is not None else None
         a.exact_varlen = 1 if (exact_varlen and duration is not None) else 0
+        a.ode_method = method
         try:
             with torch.cuda.device(y.device):
                 _lib.check(L.f5_sample(st["handle"], C.byref(a), ws.data_ptr(), ws.numel(), stream), "f5_sample")
         finally:
             self._ws_release(ws, y.device, stream)
 
-    def sample_flops(self, B, N, steps, cfg_strength) -> float:
-        return float(_lib.lib().f5_sample_flops(self.engine()["handle"], B, N, steps, float(cfg_strength)))
+    def sample_flops(self, B, N, steps, cfg_strength, ode_method="euler") -> float:
+        evals = _ode_evals(steps, _ode_method_id(ode_method))
+        return float(_lib.lib().f5_sample_flops(self.engine()["handle"], B, N, evals, float(cfg_strength)))
 
     # -- the reference's operator signature (dit.py:319-330 / unett.py:244-255) ----------------------------------
     @torch.no_grad()
@@ -390,8 +407,10 @@ class CFM(nn.Module):
         self.transformer = transformer
         self.dim = transformer.dim
         self.sigma = sigma
-        if odeint_kwargs.get("method", "euler") != "euler":
-            raise NotImplementedError("the fused CFG+Euler kernel implements method='euler' (the shipped default)")
+        method = odeint_kwargs.get("method", "euler")
+        if method not in ("euler", "midpoint"):
+            raise NotImplementedError(f"the fused CFG + ODE update kernel implements method='euler' (the shipped default) "
+                                      f"and 'midpoint', not {method!r}")
         self.odeint_kwargs = odeint_kwargs
         self.vocab_char_map = vocab_char_map
         self.use_cuda_graph = True
@@ -477,7 +496,7 @@ class CFM(nn.Module):
         trajectory = torch.empty((steps + 1, batch, n_frames, self.num_channels), device=device, dtype=torch.float32)
         self.transformer.run(y, step_cond.float().contiguous(), text.to(torch.int64).contiguous(), t.tolist(), dur32,
                              cfg_strength, trajectory=trajectory, use_graph=self.use_cuda_graph,
-                             exact_varlen=exact_varlen)
+                             exact_varlen=exact_varlen, ode_method=self.odeint_kwargs.get("method", "euler"))
         self.transformer.clear_cache()
 
         out = torch.where(cond_mask, cond, trajectory[-1].to(dtype))

@@ -162,8 +162,12 @@ typedef struct f5_engine f5_engine;
 int f5_engine_create(const f5_arch* arch, const f5_weights* weights, f5_engine** out);
 void f5_engine_destroy(f5_engine* e);
 
+/* ODE solver of the NFE loop: torchdiffeq's fixed-grid methods on the caller's grid (odeint_kwargs, cfm.py:39-42,218).
+ * Euler evaluates the backbone once per grid step, midpoint twice (at t_k and at t_k + dt/2). */
+enum { F5_ODE_EULER = 0, F5_ODE_MIDPOINT = 1 };
+
 typedef struct {
-  int B, N, nt, steps;
+  int B, N, nt, steps;       /* steps: grid steps (t has steps+1 points) */
   const long long* text;     /* device int64 [B, nt], padded with -1 (model/utils.py:99-106) */
   const float* step_cond;    /* device fp32 [B, N, mel]  (cfm.py:151-153) */
   float* y;                  /* device fp32 [B, N, mel]  in: y0 (cfm.py:196-201), out: trajectory[-1] */
@@ -172,20 +176,23 @@ typedef struct {
   float cfg_strength;        /* < 1e-5 -> single un-packed forward (cfm.py:166-177) */
   float* trajectory;         /* device fp32 [steps+1, B, N, mel] or NULL */
   int use_graph;             /* capture one NFE step into a CUDA graph and replay it */
-  float* v_out;              /* optional device fp32 [Be, N, mel]: raw backbone output of the LAST step (the value
-                                transformer(x, cond, text, time, mask, cfg_infer=...) returns, dit.py:367-370) */
+  float* v_out;              /* optional device fp32 [Be, N, mel]: raw backbone output of the LAST evaluation (the value
+                                transformer(x, cond, text, time, mask, cfg_infer=...) returns, dit.py:367-370); for
+                                midpoint that is the evaluation at t[steps-1] + dt/2 */
   int exact_varlen;          /* with duration != NULL: 1 = every sample is computed exactly as if it were ALONE in the batch
                                 with N = duration[b] — text blocks, conv position embedding and attention see nothing past
                                 the sample's end, padded tiles are skipped.  This is what a loop of B = 1 sample() calls
                                 computes (the reference's per-chunk loop, infer/utils_infer.py:540-541), in one batch.
                                 0 = the reference's batched semantics (padded rows computed; attended unless
                                 arch.attn_mask_enabled) */
+  int ode_method;            /* F5_ODE_EULER or F5_ODE_MIDPOINT; any other value is rejected (since f5_version() 101) */
 } f5_sample_args;
-size_t f5_sample_workspace_bytes(const f5_engine* e, int B, int N, int steps, float cfg_strength);
+/* `evals` below is the number of backbone evaluations of the call: steps for Euler, 2 * steps for midpoint. */
+size_t f5_sample_workspace_bytes(const f5_engine* e, int B, int N, int evals, float cfg_strength);
 int f5_sample(f5_engine* e, const f5_sample_args* args, void* workspace, size_t ws_bytes, f5_stream_t stream);
 
 /* algorithmic FLOPs of one f5_sample call (SURVEY.md §8d formula) — used by bench.py for the roofline */
-double f5_sample_flops(const f5_engine* e, int B, int N, int steps, float cfg_strength);
+double f5_sample_flops(const f5_engine* e, int B, int N, int evals, float cfg_strength);
 
 #ifdef __cplusplus
 }
